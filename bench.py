@@ -22,6 +22,9 @@ Printed JSON (one line, rank 0):
 `--impl reference` times that CPU learner alone: the reference's own AtariNet / vtrace / loss_fn modules (oracle/_ref, built by
 oracle/make_ref.py in the build container) under the learn() statements of impala_atari.py:288-346 -- the trainer module
 itself cannot be imported (SURVEY.md §0); without oracle/_ref the arm falls back to the oracle port and says so (kind).
+`--dump-outputs DIR` writes what the last timed step computed (step_outputs) as DIR/<name>.npy, float32.  That step starts from the
+seeded initial weights and a zero optimizer state and reads a seeded batch, so two builds run with the same arguments can be compared
+output for output (to the rounding of fp32 atomics).
 """
 import argparse
 import json
@@ -31,6 +34,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree, which may be read-only (no __pycache__ either)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -140,6 +144,34 @@ def make_host_pool(T, B, A, n, seed):
         hb['episode_return'].copy_(torch.from_numpy(rng.randn(T + 1, B).astype(np.float32)))
         pool.append(hb)
     return pool
+
+
+DUMP_LIMIT = 64 << 20     # bytes written by --dump-outputs at most
+
+
+def step_outputs(learner):
+    """what one learner step hands its caller: the four losses and the gradient norm of the stats dict, the V-trace targets and
+    policy-gradient advantages [T, B], the updated parameters and the step's gradients (AtariNet state_dict names)"""
+    r = learner._resdev.cpu().numpy()
+    out = {'pg_loss': r[0:1], 'baseline_loss': r[1:2], 'entropy_loss': r[2:3], 'total_loss': r[3:4], 'grad_norm': r[4:5],
+           'vs': learner._vs.cpu().numpy(), 'pg_advantages': learner._pg_adv.cpu().numpy()}
+    out.update({f'param.{n}': v.cpu().numpy() for n, v in learner.params.items()})
+    out.update({f'grad.{n}': v.cpu().numpy() for n, v in learner.grads.items()})
+    return out
+
+
+def dump_outputs(d, arrays):
+    """DIR/<name>.npy in float32.  Should the arrays exceed DUMP_LIMIT together, each large one is replaced by the same seeded
+    sample of its flattened elements (same sizes and indices in every run with the same arguments)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if total > DUMP_LIMIT and a.size > 4096:
+            keep = max(4096, a.size * DUMP_LIMIT // (2 * total))
+            a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(d, name + '.npy'), a)
 
 
 def usable_cores():
@@ -268,7 +300,10 @@ def _main(real_stdout):
     ap.add_argument('--no-extras', action='store_true', help='skip the other_configs / per_sampler measurements')
     ap.add_argument('--publish-every', type=int, default=1, help='weight publish cadence of the end-to-end loop (reference: every step)')
     ap.add_argument('--use-lstm', action='store_true', help='AtariNet(use_lstm=True) learner (BASELINE.json configs[4]: use with --T 100)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed as DIR/<name>.npy (rank 0)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
     if args.warmup < 3:
         args.warmup = 3
     rank = int(os.environ.get('RANK', '0'))
@@ -298,6 +333,7 @@ def _main(real_stdout):
     T, B, A, K, W = args.T, args.B, args.A, args.steps, args.warmup
     hp = ImpalaHParams(rollout_length=T, batch_size=B, num_actions=A, use_lstm=args.use_lstm)
     learner = B200ImpalaLearner(hp, device=dev, seed=0)
+    init_weights = learner.state_dict() if args.dump_outputs else None       # the seeded initial weights, on the device
     host_pool = make_host_pool(T, B, A, POOL, seed=rank)
     dev_pool = [{k: v.to(dev, non_blocking=True) for k, v in hb.items()} for hb in host_pool]
     torch.cuda.synchronize()
@@ -322,17 +358,27 @@ def _main(real_stdout):
     if rank == 0:
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
     for i in range(K):
+        if init_weights is not None and i == K - 1:
+            # the dumped step starts from the same state in every run: the gradient kernels sum with fp32 atomics, and over many
+            # RMSprop steps their rounding grows into a different trajectory.  The restore is excluded from the timed window.
+            r0.record()
+            learner.load_state_dict(init_weights)
+            learner.opt_state0.zero_()
+            r1.record()
         learner.learn(dev_pool[(W + i) % POOL], sync_stats=False)
     e1.record()
     barrier()
-    ms_total = max_over_ranks(e0.elapsed_time(e1))
+    ms_total = max_over_ranks(e0.elapsed_time(e1) - (r0.elapsed_time(r1) if init_weights is not None else 0.0))
     clocks = sampler.stop() if rank == 0 else None
     frames = K * T * B * world
     value = frames / (ms_total * 1e-3)
     losses_finite = bool(torch.isfinite(learner._losses).all().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_outputs(learner))
 
     # ---------------- end to end through the host-batch API ----------------
     feeder = HostBatchFeeder(learner, depth=2)

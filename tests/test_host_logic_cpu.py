@@ -1,29 +1,31 @@
 """CPU tests of the host side that mirrors the reference interface: BaseAgent surface, torch.optim-layout optimizer state,
-Timings, the ActorNet stand-in vs the reference's AtariNet (build container only: /root/reference), the reference actor
-calling convention in ImpalaTrainer.get_action, rnn-state buffers."""
+Timings, the ActorNet stand-in vs the reference's AtariNet (its outputs recorded in tests/golden/reference_cases.npz by
+oracle/make_golden.py), the reference actor calling convention in ImpalaTrainer.get_action, rnn-state buffers."""
 import os
-import sys
 import threading
 
+import numpy as np
 import pytest
 import torch
 
+from oracle import make_golden as MG
+from oracle import ref_learner as R
 from scalerl_b200.learner import (B200ImpalaLearner, ImpalaHParams, LSTM_PARAM_NAMES, PARAM_NAMES, from_torch_optimizer_state,
                                   param_shapes, reference_param_order, to_torch_optimizer_state)
 from scalerl_b200.algorithms.base import BaseAgent
 from scalerl_b200.algorithms.impala.impala_atari import ImpalaArguments, ImpalaTrainer
 from scalerl_b200.algorithms.utils.atari_model import ActorNet, SyntheticAtariEnv
 from scalerl_b200.utils.profile import Timings
+from tests.conftest import GOLDEN
 
-REF = '/root/reference'
-have_ref = os.path.isdir(os.path.join(REF, 'scalerl'))
+
+def _golden():
+    return np.load(os.path.join(GOLDEN, 'reference_cases.npz'))
 
 
 def _ref_atarinet():
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    from scalerl.algorithms.utils.atari_model import AtariNet
-    return AtariNet
+    """the reference's own AtariNet class (oracle/_ref, built by oracle/make_ref.py where the reference sources are present)"""
+    return R._load('atari_model').AtariNet
 
 
 class _Shaped(torch.nn.Module):
@@ -85,12 +87,9 @@ def test_optimizer_state_is_torch_layout(optimizer, use_lstm):
 
 
 def test_reference_param_order_is_atarinet_parameters_order():
-    if not have_ref:
-        pytest.skip('reference not mounted')
-    AtariNet = _ref_atarinet()
+    g = _golden()
     for use_lstm in (False, True):
-        net = AtariNet((4, 84, 84), 6, use_lstm=use_lstm)
-        assert [n for n, _ in net.named_parameters()] == list(reference_param_order(use_lstm))
+        assert list(g[f'param_order_lstm{int(use_lstm)}']) == list(reference_param_order(use_lstm))
 
 
 def test_timings_matches_reference_statistics():
@@ -108,55 +107,47 @@ def test_timings_matches_reference_statistics():
         assert abs(tm.stds()[k] - var ** 0.5) < 1e-9
     s = tm.summary('Batch and learn: ')
     assert s.startswith('Batch and learn: ') and 'Total:' in s and 'a:' in s and 'b:' in s
-    if have_ref:                         # same numbers as the reference's own class fed the same samples
-        import importlib.util            # by path: scalerl.utils' package __init__ imports a logger that needs colorama
-        spec = importlib.util.spec_from_file_location('ref_profile', os.path.join(REF, 'scalerl', 'utils', 'profile.py'))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        RefTimings = mod.Timings
-        r = RefTimings()
-        mine = Timings()
-        clock = [0.0]
+    # same numbers as the reference's own class fed the same samples (scalerl/utils/profile.py, recorded by oracle/make_golden.py)
+    mine = Timings()
+    import timeit
+    real = timeit.default_timer
+    try:
         for x in (0.5, 0.25, 1.0, 0.75):
-            for obj in (r, mine):
-                obj.last_time = 0.0
-            import timeit
-            real = timeit.default_timer
-            try:
-                timeit.default_timer = lambda x=x: x
-                r.time('k'); mine.time('k')
-            finally:
-                timeit.default_timer = real
-        assert abs(r.means()['k'] - mine.means()['k']) < 1e-12 and abs(r.vars()['k'] - mine.vars()['k']) < 1e-12
+            mine.last_time = 0.0
+            timeit.default_timer = lambda x=x: x
+            mine.time('k')
+    finally:
+        timeit.default_timer = real
+    ref_mean, ref_var = _golden()['timings_mean_var']
+    assert abs(ref_mean - mine.means()['k']) < 1e-12 and abs(ref_var - mine.vars()['k']) < 1e-12
 
 
 @pytest.mark.parametrize('use_lstm', [False, True])
 def test_actornet_equals_reference_atarinet(use_lstm):
     """same state_dict keys/shapes, same outputs and next state as the reference model on the actor's one-step calls"""
-    if not have_ref:
-        pytest.skip('reference not mounted')
-    AtariNet = _ref_atarinet()
+    g = _golden()
+    p = f'actor_lstm{int(use_lstm)}_'
     A = 6
-    ref = AtariNet((4, 84, 84), A, use_lstm=use_lstm)
     mine = ActorNet((4, 84, 84), A, use_lstm=use_lstm)
-    sd = ref.state_dict()
-    assert list(sd) == list(mine.state_dict()) and all(sd[k].shape == mine.state_dict()[k].shape for k in sd)
-    mine.load_state_dict(sd)
+    sd = mine.state_dict()
+    assert list(g[p + 'keys']) == list(sd) and all(tuple(g[p + 'shape_' + k]) == tuple(sd[k].shape) for k in sd)
+    mine.load_state_dict(MG.actor_weights(A, use_lstm))
+    torch.manual_seed(0)                       # SyntheticAtariEnv mixes torch.initial_seed() into its seed
     env = SyntheticAtariEnv((4, 84, 84), A, seed=3)
     out = env.reset()
-    s_ref, s_mine = ref.initial_hidden_state(1), mine.initial_hidden_state(1)
-    assert len(s_ref) == len(s_mine) and all(a.shape == b.shape for a, b in zip(s_ref, s_mine))
-    ref.eval(); mine.eval()
+    s_mine = mine.initial_hidden_state(1)
+    assert [tuple(s.shape) for s in s_mine] == [tuple(s) for s in g[p + 'state_shapes']]
+    mine.eval()
     for t in range(4):
-        with torch.no_grad():
-            o_ref, s_ref = ref(out, s_ref)
         o_mine, s_mine = mine(out, s_mine)
-        assert torch.allclose(o_ref['policy_logits'], o_mine['policy_logits'], atol=1e-5)
-        assert torch.allclose(o_ref['baseline'], o_mine['baseline'], atol=1e-5)
-        assert torch.equal(o_ref['action'], o_mine['action'])
-        for a, b in zip(s_ref, s_mine):
-            assert torch.allclose(a, b, atol=1e-5)
-        out = env.step(o_ref['action'])
+        q = f'{p}t{t}_'
+        assert torch.allclose(torch.from_numpy(g[q + 'logits']), o_mine['policy_logits'], atol=1e-5)
+        assert torch.allclose(torch.from_numpy(g[q + 'baseline']), o_mine['baseline'], atol=1e-5)
+        assert torch.equal(torch.from_numpy(g[q + 'action']), o_mine['action'])
+        assert len(s_mine) == len(g[p + 'state_shapes'])
+        for i, b in enumerate(s_mine):
+            assert torch.allclose(torch.from_numpy(g[f'{q}state{i}']), b, atol=1e-5)
+        out = env.step(o_mine['action'])
         if t == 1:
             out['done'] = torch.ones(1, 1, dtype=torch.bool)          # exercise the state reset (atari_model.py:114-116)
 
@@ -166,8 +157,8 @@ def test_get_action_fills_slots_with_the_reference_actor_convention(which, tmp_p
     """ImpalaTrainer.get_action drives actor_model(env_output, agent_state) -> (outputs, state) (impala_atari.py:177-197)
     -- with the stand-in ActorNet and with the reference's own AtariNet, unchanged -- and writes rollouts + initial LSTM
     states into the shared slots"""
-    if which != 'actornet' and not have_ref:
-        pytest.skip('reference not mounted')
+    if which != 'actornet' and not R.available():
+        pytest.skip('oracle/_ref not built (python oracle/make_ref.py, needs the reference sources)')
     use_lstm = which == 'reference_lstm'
     a = ImpalaArguments(num_actors=1, batch_size=2, rollout_length=3, num_buffers=3, use_lstm=use_lstm, output_dir=str(tmp_path))
     fn = None

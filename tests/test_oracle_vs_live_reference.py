@@ -1,9 +1,7 @@
-"""Oracle vs the REFERENCE's own modules, live and randomised -- only where /root/reference exists (the build container);
-skipped on the GPU box, where the committed goldens (tests/golden/, oracle/make_golden.py) carry the pin.
-
-Loads the leaf modules of the hot path by file path (the package itself cannot be imported, SURVEY.md §0):
-scalerl/algorithms/impala/vtrace.py, loss_fn.py and scalerl/algorithms/utils/atari_model.py."""
-import importlib.util
+"""Oracle vs the REFERENCE's own modules on randomised inputs: the reference's outputs are stored in
+tests/golden/reference_cases.npz, recorded by oracle/make_golden.py from scalerl/algorithms/impala/vtrace.py, loss_fn.py,
+scalerl/algorithms/utils/atari_model.py and scalerl/data/segment_tree.py.  The inputs are rebuilt from the same seeds by the
+input functions of oracle/make_golden.py."""
 import os
 
 import numpy as np
@@ -11,147 +9,88 @@ import pytest
 import torch
 
 from oracle import impala_oracle as O
-
-REF = '/root/reference/scalerl/algorithms'
-pytestmark = pytest.mark.skipif(not os.path.exists(f'{REF}/impala/vtrace.py'), reason='reference tree not present')
-
-
-def _load(name, path):
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+from oracle import make_golden as MG
+from tests.conftest import GOLDEN
 
 
 @pytest.fixture(scope='module')
 def ref():
-    return dict(vtrace=_load('live_ref_vtrace', f'{REF}/impala/vtrace.py'), loss_fn=_load('live_ref_loss_fn', f'{REF}/impala/loss_fn.py'),
-                atari_model=_load('live_ref_atari_model', f'{REF}/utils/atari_model.py'))
+    return np.load(os.path.join(GOLDEN, 'reference_cases.npz'))
 
 
 @pytest.mark.parametrize('seed', range(12))
 def test_vtrace_from_logits_random_shapes(ref, seed):
     """vtrace.py:43-172 on random (T, B, A), with terminal steps and every clip-threshold combination incl. None"""
-    rng = np.random.RandomState(100 + seed)
-    T, B, A = int(rng.randint(1, 40)), int(rng.randint(1, 9)), int(rng.randint(1, 19))
-    cr = [1.0, None, 2.5, 0.3][seed % 4]
-    cp = [1.0, 0.7, None][seed % 3]
-    t = lambda *s: torch.from_numpy(rng.randn(*s).astype(np.float32))
-    bl, tl = t(T, B, A) * 1.5, t(T, B, A) * 1.5
-    actions = torch.from_numpy(rng.randint(0, A, size=(T, B)).astype(np.int64))
-    discounts = torch.from_numpy(((rng.rand(T, B) > 0.15) * 0.99).astype(np.float32))
-    rewards, values, boot = t(T, B), t(T, B), t(B)
-    r = ref['vtrace'].from_logits(behavior_policy_logits=bl, target_policy_logits=tl, actions=actions, discounts=discounts, rewards=rewards,
-                                  values=values, bootstrap_value=boot, clip_rho_threshold=cr, clip_pg_rho_threshold=cp)
-    vs, pg, lr, balp, talp = O.vtrace_from_logits(bl, tl, actions, discounts, rewards, values, boot, cr, cp)
-    assert torch.allclose(vs, r.vs, rtol=1e-5, atol=1e-5) and torch.allclose(pg, r.pg_advantages, rtol=1e-5, atol=1e-5)
-    assert torch.allclose(lr, r.log_rhos, atol=1e-6) and torch.allclose(balp, r.behavior_action_log_probs, atol=1e-6)
-    assert torch.allclose(talp, r.target_action_log_probs, atol=1e-6)
+    a = MG.vtrace_random_inputs(seed)
+    r = {k: torch.from_numpy(ref[f'vtrace_s{seed}_{k}']) for k in ('vs', 'pg', 'log_rhos', 'balp', 'talp')}
+    cr, cp = a['clip_rho_threshold'], a['clip_pg_rho_threshold']
+    discounts, rewards, values, boot = a['discounts'], a['rewards'], a['values'], a['bootstrap_value']
+    vs, pg, lr, balp, talp = O.vtrace_from_logits(a['behavior_policy_logits'], a['target_policy_logits'], a['actions'], discounts, rewards,
+                                                  values, boot, cr, cp)
+    assert torch.allclose(vs, r['vs'], rtol=1e-5, atol=1e-5) and torch.allclose(pg, r['pg'], rtol=1e-5, atol=1e-5)
+    assert torch.allclose(lr, r['log_rhos'], atol=1e-6) and torch.allclose(balp, r['balp'], atol=1e-6)
+    assert torch.allclose(talp, r['talp'], atol=1e-6)
     # the float64 scalar witness agrees with both
     vs64, pg64 = O.vtrace_from_importance_weights_np64(lr.numpy(), discounts.numpy(), rewards.numpy(), values.numpy(), boot.numpy(), cr, cp)
-    assert np.allclose(vs64, r.vs.numpy(), rtol=1e-4, atol=1e-4) and np.allclose(pg64, r.pg_advantages.numpy(), rtol=1e-4, atol=1e-4)
+    assert np.allclose(vs64, r['vs'].numpy(), rtol=1e-4, atol=1e-4) and np.allclose(pg64, r['pg'].numpy(), rtol=1e-4, atol=1e-4)
 
 
 @pytest.mark.parametrize('seed', range(6))
 def test_losses_and_head_gradients_random(ref, seed):
     """loss_fn.py:5-23 with the weights of impala_atari.py:320-330; the oracle's closed-form head gradients equal autograd
     through the reference's loss functions"""
-    rng = np.random.RandomState(200 + seed)
-    T, B, A = int(rng.randint(1, 25)), int(rng.randint(1, 7)), int(rng.randint(2, 19))
-    bc, ec = 0.5, 0.0006 * (1 + seed)
-    logits = torch.from_numpy(rng.randn(T, B, A).astype(np.float32)).requires_grad_(True)
-    values = torch.from_numpy(rng.randn(T, B).astype(np.float32)).requires_grad_(True)
-    actions = torch.from_numpy(rng.randint(0, A, size=(T, B)).astype(np.int64))
-    vs = torch.from_numpy(rng.randn(T, B).astype(np.float32))
-    adv = torch.from_numpy(rng.randn(T, B).astype(np.float32))
-    L = ref['loss_fn']
-    pg = L.compute_policy_gradient_loss(logits, actions, adv)
-    bl = bc * L.compute_baseline_loss(vs - values)
-    en = ec * L.compute_entropy_loss(logits)
-    (pg + bl + en).backward()
-    o_pg, o_bl, o_en = O.impala_losses(logits.detach(), actions, values.detach(), vs, adv, bc, ec)
-    pg, bl, en = pg.detach(), bl.detach(), en.detach()
-    assert abs(float(o_pg) - float(pg)) <= 1e-4 * max(1, abs(float(pg))) and abs(float(o_bl) - float(bl)) <= 1e-4 * max(1, abs(float(bl)))
-    assert abs(float(o_en) - float(en)) <= 1e-5 * max(1, abs(float(en)))
-    dl, dv = O.head_grads(logits.detach(), actions, values.detach(), vs, adv, bc, ec)
-    assert torch.allclose(dl, logits.grad, rtol=1e-4, atol=1e-6) and torch.allclose(dv, values.grad, rtol=1e-5, atol=1e-6)
+    logits, values, actions, vs, adv, bc, ec = MG.loss_random_inputs(seed)
+    pg, bl, en = (float(x) for x in ref[f'loss_s{seed}_losses'])
+    o_pg, o_bl, o_en = O.impala_losses(logits, actions, values, vs, adv, bc, ec)
+    assert abs(float(o_pg) - pg) <= 1e-4 * max(1, abs(pg)) and abs(float(o_bl) - bl) <= 1e-4 * max(1, abs(bl))
+    assert abs(float(o_en) - en) <= 1e-5 * max(1, abs(en))
+    dl, dv = O.head_grads(logits, actions, values, vs, adv, bc, ec)
+    assert torch.allclose(dl, torch.from_numpy(ref[f'loss_s{seed}_dlogits']), rtol=1e-4, atol=1e-6)
+    assert torch.allclose(dv, torch.from_numpy(ref[f'loss_s{seed}_dvalues']), rtol=1e-5, atol=1e-6)
 
 
 @pytest.mark.parametrize('A,seed', [(6, 0), (18, 1), (3, 2)])
 def test_atarinet_forward_random_weights(ref, A, seed):
     """atari_model.py:77-143 (no LSTM): the oracle's functional forward == AtariNet.forward with the same state_dict,
     greedy actions excluded (the reference samples with torch.multinomial in training mode)"""
-    net = ref['atari_model'].AtariNet((4, 84, 84), A, use_lstm=False)
     params = O.init_params(A, seed=seed)
-    net.load_state_dict(params)
     T, B = 3, 2
     batch = O.synthetic_batch(T, B, A, seed=seed)
-    with torch.no_grad():
-        out, _ = net(batch, ())                      # the reference reads inputs['action'] as the last action (SURVEY.md §0.9)
     lg, bs = O.atari_forward(params, batch['obs'], batch['reward'], batch['action'])
-    assert torch.allclose(lg.view(T + 1, B, A), out['policy_logits'], rtol=1e-4, atol=1e-5)
-    assert torch.allclose(bs.view(T + 1, B), out['baseline'], rtol=1e-4, atol=1e-5)
+    assert torch.allclose(lg.view(T + 1, B, A), torch.from_numpy(ref[f'atari_a{A}_s{seed}_logits']), rtol=1e-4, atol=1e-5)
+    assert torch.allclose(bs.view(T + 1, B), torch.from_numpy(ref[f'atari_a{A}_s{seed}_baseline']), rtol=1e-4, atol=1e-5)
 
 
 @pytest.mark.parametrize('seed', range(6))
-def test_per_trees_random_against_reference_segment_trees(seed):
+def test_per_trees_random_against_reference_segment_trees(ref, seed):
     """scalerl/data/segment_tree.py driven by the statements of PrioritizedReplayBuffer (replay_buffer.py:318-381) vs the
     PER oracle: random capacities (incl. wrap-around of the ring pointer), duplicate update indices, several rounds"""
     from oracle.per_oracle import PerOracle
-    seg = _load('live_ref_segment_tree', '/root/reference/scalerl/data/segment_tree.py')
-    rng = np.random.RandomState(300 + seed)
-    mem = int(rng.choice([7, 64, 100, 333, 1024]))
-    alpha, beta = float(rng.choice([0.4, 0.6, 1.0])), float(rng.choice([0.4, 0.7, 1.0]))
-    cap = 1
-    while cap < mem:
-        cap *= 2
-    st, mt = seg.SumSegmentTree(cap), seg.MinSegmentTree(cap)
+    mem, alpha, beta, rounds = MG.per_random_inputs(seed)
     o = PerOracle(mem, alpha)
-    max_p, ptr, size = 1.0, 0, 0
-    for rnd in range(3):
-        nadd = int(rng.randint(1, 2 * mem))
-        for _ in range(nadd):
-            st[ptr] = max_p ** alpha
-            mt[ptr] = max_p ** alpha
-            ptr = (ptr + 1) % mem
-            size = min(size + 1, mem)
+    max_p, size = 1.0, 0
+    for rnd, (nadd, idx, pr, u) in enumerate(rounds):
         o.add(nadd)
-        k = int(rng.randint(1, 50))
-        idx = rng.randint(0, size, size=k)                       # duplicates on purpose: last write wins
-        pr = rng.rand(k) * 4 + 1e-3
-        for i, p in zip(idx, pr):
-            st[int(i)] = float(p) ** alpha
-            mt[int(i)] = float(p) ** alpha
-            max_p = max(max_p, float(p))
+        size = min(size + nadd, mem)
         o.update_priorities(idx, pr)
-        batch = int(rng.randint(1, 40))
-        u = rng.rand(batch)
-        p_total = st.sum(0, size - 1)
-        segment = p_total / batch
-        want = [st.find_prefixsum_idx(segment * i + (segment * (i + 1) - segment * i) * float(u[i])) for i in range(batch)]
-        p_min = mt.min() / st.sum()
-        max_w = (p_min * size) ** (-beta)
-        want_w = [((st[i] / st.sum()) * size) ** (-beta) / max_w for i in want]
+        max_p = max(max_p, float(pr.max()))
         got, got_w = o.sample(u, beta)
-        assert np.array_equal(got, np.array(want, dtype=np.int64)), (seed, rnd)
-        assert np.array_equal(got_w, np.array(want_w, dtype=np.float64))
-        assert o.size == size and o.max_priority == max_p and o.sum_tree.operate() == st.sum() and o.min_tree.operate() == mt.min()
+        p = f'per_s{seed}_r{rnd}_'
+        assert np.array_equal(got, ref[p + 'idx']), (seed, rnd)
+        assert np.array_equal(got_w, ref[p + 'w'])
+        assert o.size == size and o.max_priority == max_p
+        assert o.sum_tree.operate() == ref[p + 'sum'][0] and o.min_tree.operate() == ref[p + 'min'][0]
 
 
 @pytest.mark.parametrize('A,seed', [(6, 0), (3, 1)])
 def test_atarinet_lstm_forward_random(ref, A, seed):
     """use_lstm=True (atari_model.py:52-55,109-120): the oracle's step-wise 2-layer LSTM with done-resets and a random
     initial state vs the reference module holding the same weights"""
-    net = ref['atari_model'].AtariNet((4, 84, 84), A, use_lstm=True)
-    params, lp = O.init_params(A, seed=seed), O.init_lstm_params(A, seed=seed)
-    net.load_state_dict({**params, **lp})
-    T, B = 4, 3
-    batch = O.synthetic_batch(T, B, A, seed=seed + 7, done_p=0.3)
-    g = torch.Generator().manual_seed(seed)
-    state = (torch.randn(2, B, 513 + A, generator=g) * 0.1, torch.randn(2, B, 513 + A, generator=g) * 0.1)
+    params, lp, batch, state = MG.lstm_random_inputs(A, seed)
+    T, B = batch['reward'].shape[0] - 1, batch['reward'].shape[1]
     with torch.no_grad():
-        out, ns = net(batch, state)
         lg, bs, os_ = O.atari_forward_lstm(params, lp, batch['obs'], batch['reward'], batch['action'], batch['done'], state)
-    assert torch.allclose(lg.view(T + 1, B, A), out['policy_logits'], rtol=1e-4, atol=1e-5)
-    assert torch.allclose(bs.view(T + 1, B), out['baseline'], rtol=1e-4, atol=1e-5)
-    assert torch.allclose(os_[0], ns[0], rtol=1e-4, atol=1e-5) and torch.allclose(os_[1], ns[1], rtol=1e-4, atol=1e-5)
+    r = {k: torch.from_numpy(ref[f'lstm_a{A}_s{seed}_{k}']) for k in ('logits', 'baseline', 'h', 'c')}
+    assert torch.allclose(lg.view(T + 1, B, A), r['logits'], rtol=1e-4, atol=1e-5)
+    assert torch.allclose(bs.view(T + 1, B), r['baseline'], rtol=1e-4, atol=1e-5)
+    assert torch.allclose(os_[0], r['h'], rtol=1e-4, atol=1e-5) and torch.allclose(os_[1], r['c'], rtol=1e-4, atol=1e-5)
