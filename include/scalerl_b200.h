@@ -125,9 +125,8 @@ int64_t srl_learner_workspace_bytes(const srl_learner_t* L);
 /* update a hyper-parameter that does not change buffer sizes (lr, costs, clip...) */
 int srl_learner_set_config(srl_learner_t* L, const srl_config_t* cfg);
 
-/* run-time switches of one learner context: "column_fusion" (default 1; 0 = three kernels head_fwd / impala_tail / head_bwd
- * instead of the fused column kernel -- the environment variable SRL_NO_COLUMN_FUSION is read once, at creation);
- * "fused_fwd" (default 0, SRL_FUSED_FWD=1): u8 frame conversion + conv1 + conv2 as ONE persistent kernel (bf16 mode) instead of three. */
+/* run-time switch of one learner context: "column_fusion" (default 1; 0 = three kernels head_fwd / impala_tail / head_bwd
+ * instead of the fused column kernel -- the environment variable SRL_NO_COLUMN_FUSION is read once, at creation). */
 int srl_learner_set_option(srl_learner_t* L, const char* name, int value);
 
 /* optimizer step count (Adam's bias-correction t; torch.optim state['step']): restore it when resuming from a checkpoint

@@ -193,7 +193,6 @@ struct srl_learner {
   float *core, *lstm_out, *dout, *dcore;   // [NF][H], [NF][H], [NB][H], [NB][H]
   char* lstm_arena;
   int64_t lstm_off0, lstm_len;    // LSTM gradient range inside the flat buffer
-  bool fused_front;               // frame conversion + conv1 + conv2 as one kernel (SRL_FUSED_FWD / srl_learner_set_option "fused_fwd")
   bool column_fusion;             // heads + V-trace/loss + dh in one column kernel (SRL_NO_COLUMN_FUSION / srl_learner_set_option)
   Profiler pf;                    // per-kernel event bracketing (off by default)
   cudaEvent_t events[2 * PS_COUNT];
@@ -202,7 +201,7 @@ struct srl_learner {
 
 static const char* kSlotNames[PS_COUNT] = {"obs_s2d", "conv1_fwd", "conv2_fwd", "conv3_fwd", "fc_fwd", "head_fwd", "vtrace_loss_tail",
                                            "zero_grads", "head_bwd", "fc_wgrad", "fc_dgrad", "conv3_wgrad", "conv3_dgrad", "conv2_wgrad",
-                                           "conv2_dgrad", "conv1_wgrad", "conv_wgrad_finalize", "grad_norm", "optimizer", "pack_weights", "enc_fused_fwd"};
+                                           "conv2_dgrad", "conv1_wgrad", "conv_wgrad_finalize", "grad_norm", "optimizer", "pack_weights"};
 
 static int check_cfg(const srl_config_t* c) {
   REQ(c, "config is NULL");
@@ -216,7 +215,6 @@ static int check_cfg(const srl_config_t* c) {
   return 0;
 }
 
-static int pack_priority(int least, int greatest);
 extern "C" int srl_learner_create(const srl_config_t* cfg, float* params, float* grads, float* opt0, float* opt1, srl_learner_t** out) {
   int rc = check_cfg(cfg);
   if (rc) return rc;
@@ -234,9 +232,6 @@ extern "C" int srl_learner_create(const srl_config_t* cfg, float* params, float*
   L->G = make_ptrs(grads, cfg->A);
   L->step = 0; L->have_fwd = false;
   { const char* nf = getenv("SRL_NO_COLUMN_FUSION"); L->column_fusion = !(nf && atoi(nf) != 0); }   // read once, at creation
-  // measured (profiles/r02_fused_front_timeline.md): one CTA per SM with ONE MMA-issuing thread paces the fused front at ~10 us per
-  // frame -- 52 us against 47 us for the three kernels it replaces -- so it is opt-in until it issues from two warps
-  { const char* ff = getenv("SRL_FUSED_FWD"); L->fused_front = ff && atoi(ff) != 0; }
   for (int i = 0; i < 2 * PS_COUNT; ++i) L->events[i] = nullptr;
   for (int i = 0; i < PS_COUNT; ++i) L->slot_used[i] = false;
   const int64_t NF = (int64_t)(cfg->T + 1) * cfg->B, NB = (int64_t)cfg->T * cfg->B, A = cfg->A;
@@ -296,9 +291,11 @@ extern "C" int srl_learner_create(const srl_config_t* cfg, float* params, float*
       cudaStreamCreateWithFlags(&L->ss.side2, cudaStreamNonBlocking) != cudaSuccess ||
       cudaStreamCreateWithFlags(&L->ss.side3, cudaStreamNonBlocking) != cudaSuccess) L->ss.side = nullptr;
   {
+    // the re-pack stream sits one level BELOW the greatest priority (which the learner's capture stream uses for the main chain) and above the
+    // wgrad streams (default = least): its short blocks fill the slots the frame conversion leaves free without delaying it
     int lo = 0, hi = 0;       // (numerically lowest = greatest priority)
     if (L->ss.side && (cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess ||
-                       cudaStreamCreateWithPriority(&L->ss.pack, cudaStreamNonBlocking, pack_priority(lo, hi)) != cudaSuccess)) L->ss.side = nullptr;
+                       cudaStreamCreateWithPriority(&L->ss.pack, cudaStreamNonBlocking, hi + 1 > lo ? lo : hi + 1) != cudaSuccess)) L->ss.side = nullptr;
   }
   for (int e2 = 0; e2 < 12 && L->ss.side; ++e2)
     if (cudaEventCreateWithFlags(&L->ss.ev[e2], cudaEventDisableTiming) != cudaSuccess) { L->ss.side = nullptr; }
@@ -400,7 +397,6 @@ extern "C" int srl_learner_set_config(srl_learner_t* L, const srl_config_t* cfg)
 extern "C" int srl_learner_set_option(srl_learner_t* L, const char* name, int value) {
   REQ(L && name, "set_option: NULL argument");
   if (strcmp(name, "column_fusion") == 0) { L->column_fusion = value != 0; return 0; }
-  if (strcmp(name, "fused_fwd") == 0) { L->fused_front = value != 0; return 0; }
   return fail(SRL_EINVAL, "set_option: unknown option '%s'", name);
 }
 
@@ -439,29 +435,13 @@ int pdl_skip_mask() {
 }
 }  // namespace srl
 
-// the re-pack stream sits one level BELOW the greatest priority (which the learner's capture stream uses for the main chain) and above the wgrad
-// streams (default = least): its short blocks fill the slots the frame conversion leaves free without delaying it.  SRL_PACK_PRIORITY overrides.
-static int pack_priority(int least, int greatest) {
-  const char* e = getenv("SRL_PACK_PRIORITY");
-  int v = e ? atoi(e) : greatest + 1;
-  if (v < greatest) v = greatest;
-  if (v > least) v = least;
-  return v;
-}
-
 static int encode_impl(srl_learner* L, const uint8_t* obs, int frames, cudaStream_t st, bool zero_small_grads = false) {
-  const bool zero_small_grads_in = zero_small_grads;      // true = called from the learner step (forward + backward)
+  // zero_small_grads: true when called from the learner step (forward + backward)
   L->pf.st = st;
   pdl_set_active(!L->pf.on);
   // The bf16 operand copies are re-derived from the fp32 master weights at the START of every forward (not at the end
   // of the optimizer step): the pack kernel runs on the side stream underneath the frame conversion.
   cudaEvent_t packed = nullptr;
-  if (zero_small_grads && (side_mode() & 4)) {
-    int64_t off[12], cnt[12];
-    layout(L->cfg.A, off, cnt);
-    CU(cudaMemsetAsync(L->grads, 0, off[6] * sizeof(float), st), "zero small grads");
-    zero_small_grads = false;
-  }
   if (L->ss.side && !L->pf.on) {
     CU(cudaEventRecord(L->ss.ev[5], st), "fork pack");
     CU(cudaStreamWaitEvent(L->ss.pack, L->ss.ev[5], 0), "fork pack");
@@ -485,11 +465,11 @@ static int encode_impl(srl_learner* L, const uint8_t* obs, int frames, cudaStrea
     CU(launch_pack_weights(L->P, L->buf.wpack, st, L->buf.wpack_lo, true), "pack_weights");
     L->pf.e(PS_PACK);
   }
-  CU(encoder_forward(obs, frames, L->P, L->buf, L->maps, L->cfg.precision, st, L->pf, packed, &L->maps_lo, L->fused_front), "encoder_forward");
+  CU(encoder_forward(obs, frames, L->P, L->buf, L->maps, L->cfg.precision, st, L->pf, packed, &L->maps_lo), "encoder_forward");
   // learner step (bf16 mode): a3 -> fc.weight column order for the fc weight-gradient GEMM, on the wgrad side stream right after the fc forward,
   // i.e. under the column kernel (32 CTAs, the GPU is otherwise idle) instead of in the crowded backward phase
   L->buf.a3t_ready = false;
-  if (zero_small_grads_in && L->ss.side && !L->pf.on && L->cfg.precision == 0 && L->buf.a3t && !L->cfg.use_lstm) {
+  if (zero_small_grads && L->ss.side && !L->pf.on && L->cfg.precision == 0 && L->buf.a3t && !L->cfg.use_lstm) {
     CU(cudaEventRecord(L->ss.ev[10], st), "fork a3 transpose");
     CU(cudaStreamWaitEvent(L->ss.side, L->ss.ev[10], 0), "fork a3 transpose");
     CU(launch_a3_transpose(L->buf.a3, L->buf.a3t, L->cfg.T * L->cfg.B, L->ss.side), "a3_transpose");
@@ -546,7 +526,7 @@ static int fb_begin(srl_learner* L, const uint8_t* obs, const float* reward, con
   }
   L->pf.b(PS_HEAD_BWD);
   {
-    const bool fork = L->ss.side != nullptr && !L->pf.on && !(side_mode() & 2);
+    const bool fork = L->ss.side != nullptr && !L->pf.on;
     cudaStream_t sw = fork ? L->ss.side : st;
     if (fork) { CU(cudaEventRecord(L->ss.ev[8], st), "fork head wgrad"); CU(cudaStreamWaitEvent(sw, L->ss.ev[8], 0), "fork head wgrad"); }
     CU(launch_head_bwd(L->dlogits, L->dbaseline, L->buf.h, reward, action, L->P.wp, L->P.wb, NB, c.A, L->buf.dh, L->G.wp, L->G.bp, L->G.wb,
@@ -750,7 +730,6 @@ extern "C" int srl_learner_debug_buffer(srl_learner_t* L, const char* name, void
       {"logits", L->logits, NF * A}, {"baseline", L->baseline, NF}, {"dlogits", L->dlogits, NB * A}, {"dbaseline", L->dbaseline, NB},
       {"dh", L->buf.dh, NB * 512}, {"da3", L->buf.da3, NB * 81 * 64}, {"da2", L->buf.da2, NB * 100 * 64},
       {"da1", L->buf.da1, NB * 441 * 32}, {"wpack", L->buf.wpack, WPack::TOTAL},
-      {"fused_dbg", g_fused_dbg, 5 * 8 * 8 * 4},        // u64 stamps, counted in bf16 units by the Python helper (x4)
       {"a1_lo", L->buf.a1_lo, NF * 400 * 32}, {"a2_lo", L->buf.a2_lo, NF * 81 * 64}, {"a3_lo", L->buf.a3_lo, NF * 49 * 64},
       {"dh_lo", L->buf.dh_lo, NB * 512}, {"da3_lo", L->buf.da3_lo, NB * 81 * 64}, {"da2_lo", L->buf.da2_lo, NB * 100 * 64},
       {"da1_lo", L->buf.da1_lo, NB * 441 * 32}, {"wpack_lo", L->buf.wpack_lo, WPack::TOTAL}};

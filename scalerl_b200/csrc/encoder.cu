@@ -2,10 +2,8 @@
 #include "encoder_problems.cuh"
 #include "tma_problems.cuh"
 #include "res_problems.cuh"
-#include "enc_fused.cuh"
 #include "kernels.h"
 #include <initializer_list>
-#include <stdlib.h>
 
 namespace srl {
 
@@ -95,10 +93,8 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(ParamPtrs p, bf16* __
 }
 
 // u8 NCHW frames -> space-to-depth bf16 NHWC: xs[n][Y][X][c*16+dy*4+dx] = obs[n][c][4Y+dy][4X+dx]  (exact: u8 fits bf16).
-// One block per (frame, S2D_Y consecutive Y): the 16 S2D_Y source rows (c,dy) are read coalesced (21 u32 each, all loads of a
-// thread in flight together) into shared memory, then each thread converts u32 (4 x dx) -> 4 bf16 and the block writes
-// S2D_Y x 21 x 128 B contiguously.  S2D_Y = 21 (a whole frame per block, 84 B of loads in flight per thread) by default.
-template <int S2D_Y>
+// One block per frame: the 16 x 21 source rows (c,dy) are read coalesced (21 u32 each, all 84 B of loads of a thread in flight
+// together) into shared memory, then each thread converts u32 (4 x dx) -> 4 bf16 and the block writes 21 x 21 x 128 B contiguously.
 __global__ void __launch_bounds__(352) obs_s2d_kernel(const uint8_t* __restrict__ obs, bf16* __restrict__ xs, int frame_blocks,
                                                       const float* __restrict__ w1, bf16* __restrict__ w1k, bf16* __restrict__ w1k_lo) {
   pdl_wait(1);     // launched with programmatic stream serialization: see common.cuh
@@ -114,26 +110,26 @@ __global__ void __launch_bounds__(352) obs_s2d_kernel(const uint8_t* __restrict_
     }
     return;
   }
-  __shared__ uint32_t tile[S2D_Y][16][21];
-  const int n = blockIdx.x / (21 / S2D_Y), Y0 = (blockIdx.x - n * (21 / S2D_Y)) * S2D_Y;
+  __shared__ uint32_t tile[21][16][21];
+  const int n = blockIdx.x;
   const int t = threadIdx.x;
   if (t < 336) {
     const int g = t / 21, X = t - g * 21;      // g = (c, dy)
     const uint8_t* src = obs + (size_t)n * 28224 + (g >> 2) * 7056 + (g & 3) * 84;
 #pragma unroll
-    for (int y = 0; y < S2D_Y; ++y) tile[y][g][X] = __ldg(reinterpret_cast<const uint32_t*>(src + (Y0 + y) * 336) + X);
+    for (int y = 0; y < 21; ++y) tile[y][g][X] = __ldg(reinterpret_cast<const uint32_t*>(src + y * 336) + X);
   }
   __syncthreads();
   if (t < 336) {
     const int X = t >> 4, g = t & 15;
 #pragma unroll
-    for (int y = 0; y < S2D_Y; ++y) {
+    for (int y = 0; y < 21; ++y) {
       const uint32_t w = tile[y][g][X];
       const float f0 = __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7540)) - 8388608.f;
       const float f1 = __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7541)) - 8388608.f;
       const float f2 = __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7542)) - 8388608.f;
       const float f3 = __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7543)) - 8388608.f;
-      *reinterpret_cast<uint2*>(xs + (((size_t)n * 21 + Y0 + y) * 21 + X) * 64 + g * 4) = make_uint2(pack_bf16x2(f0, f1), pack_bf16x2(f2, f3));
+      *reinterpret_cast<uint2*>(xs + (((size_t)n * 21 + y) * 21 + X) * 64 + g * 4) = make_uint2(pack_bf16x2(f0, f1), pack_bf16x2(f2, f3));
     }
   }
 }
@@ -290,39 +286,19 @@ cudaError_t build_tma_maps_lo(const EncoderBuffers& b, int NF, int NB, TmaMapsLo
   return ok ? cudaSuccess : cudaErrorInvalidValue;
 }
 
-unsigned long long* g_fused_dbg = nullptr;
 static cudaError_t launch_s2d(const uint8_t* obs, int frames, bf16* xs, cudaStream_t st, const float* w1, bf16* w1k, bf16* w1k_lo) {
-  static const int ygroup = [] { const char* e = getenv("SRL_S2D_Y"); const int v = e ? atoi(e) : 21; return (v == 3 || v == 7) ? v : 21; }();
   constexpr int WB = (32 * 256 + 351) / 352;      // extra blocks that write conv1's weight copy
-  if (ygroup == 3) SRL_TRY(launch_chain<PDL_SIMT>(obs_s2d_kernel<3>, dim3(frames * 7 + WB), dim3(352), 0, st, obs, xs, frames * 7, w1, w1k, w1k_lo));
-  else if (ygroup == 7) SRL_TRY(launch_chain<PDL_SIMT>(obs_s2d_kernel<7>, dim3(frames * 3 + WB), dim3(352), 0, st, obs, xs, frames * 3, w1, w1k, w1k_lo));
-  else SRL_TRY(launch_chain<PDL_SIMT>(obs_s2d_kernel<21>, dim3(frames + WB), dim3(352), 0, st, obs, xs, frames, w1, w1k, w1k_lo));
+  SRL_TRY(launch_chain<PDL_SIMT>(obs_s2d_kernel, dim3(frames + WB), dim3(352), 0, st, obs, xs, frames, w1, w1k, w1k_lo));
   return cudaGetLastError();
 }
 
-// persistent CTAs of the resident-window kernels: one per SM by default; data-parallel runs leave a few SMs to the NCCL
-// all-reduce that overlaps the conv backward (SRL_PERSISTENT_CTAS, read once)
-static int persistent_ctas() {
-  static int v = 0;
-  if (!v) {
-    const char* e = getenv("SRL_PERSISTENT_CTAS");
-    v = e ? atoi(e) : 148;
-    if (v < 16 || v > 148) v = 148;
-  }
-  return v;
-}
-#define kPersistentCtas persistent_ctas()
+// persistent CTAs of the resident-window kernels: one per SM
+constexpr int kPersistentCtas = 148;
 // persistent CTAs of the backward chain's resident-window kernels (conv3 / conv2 dgrad, conv1 wgrad): fewer than one per SM leaves SMs to the
-// lower-priority side-stream wgrads while the chain runs.  SRL_BWD_CTAS overrides (diagnostics).
-static int bwd_ctas() {
-  static const int v = [] { const char* e = getenv("SRL_BWD_CTAS"); int x = e ? atoi(e) : 0; return x < 16 || x > 148 ? 0 : x; }();
-  return v ? v : persistent_ctas() - persistent_ctas() / 9;      // 132 of 148: measured -1.5 us per step at T=20, B=32 (148: 0.1607, 132: 0.1591, 120: 0.1629 ms)
-}
-// CTAs of the conv3 / conv2 weight-gradient kernels (side streams).  SRL_WGRAD_CTAS overrides (diagnostics).
-static int side_wgrad_ctas() {
-  static const int v = [] { const char* e = getenv("SRL_WGRAD_CTAS"); int x = e ? atoi(e) : 64; return x < 8 || x > 148 ? 64 : x; }();
-  return v;
-}
+// lower-priority side-stream wgrads while the chain runs.  132 of 148: measured -1.5 us per step at T=20, B=32 (148: 0.1607, 132: 0.1591, 120: 0.1629 ms)
+constexpr int kBwdCtas = 132;
+// CTAs of the conv3 / conv2 weight-gradient kernels (side streams)
+constexpr int kSideWgradCtas = 64;
 
 // workspace [tap-block][row][co] -> PyTorch-layout conv weight gradients (plain stores), and re-zero what was read
 __global__ void __launch_bounds__(256) conv_wgrad_finalize_kernel(float* __restrict__ ws, float* __restrict__ g1, float* __restrict__ g2,
@@ -346,35 +322,19 @@ __global__ void __launch_bounds__(256) conv_wgrad_finalize_kernel(float* __restr
 }
 
 cudaError_t encoder_forward(const uint8_t* obs, int frames, const ParamPtrs& p, const EncoderBuffers& buf, const TmaMaps& maps, int mode,
-                            cudaStream_t st, const Profiler& pf, cudaEvent_t wait_before_conv1, const TmaMapsLo* lo, bool fused_front) {
+                            cudaStream_t st, const Profiler& pf, cudaEvent_t wait_before_conv1, const TmaMapsLo* lo) {
   if (frames <= 0) return cudaSuccess;
   if ((mode != 0 && mode != 1) || !maps.valid) return cudaErrorInvalidValue;
   const int sp = mode;                                    // 1: fp32-accurate split operands
   TmaMapsLo dummy;                                        // bf16 mode: the low maps are never touched by the kernels
   if (sp && (!lo || !lo->valid)) return cudaErrorInvalidValue;
   const TmaMapsLo& L = sp ? *lo : dummy;
-  // bf16 mode: frame conversion + conv1 + conv2 as ONE persistent kernel (enc_fused.cuh); SRL_FUSED_FWD=0 or the fp32-accurate
-  // operand mode use the three separate kernels
-  if (fused_front && !sp && (reinterpret_cast<uintptr_t>(obs) & 15) == 0) {
-    static unsigned long long* dbg_buf = [] {       // SRL_FUSED_DEBUG=1: CTA 0 stamps its phases (tests/diag/diag_fused.py prints them)
-      const char* e = getenv("SRL_FUSED_DEBUG");
-      unsigned long long* q = nullptr;
-      if (e && atoi(e) != 0 && cudaMalloc(&q, 5 * FF_DBG_FRAMES * FF_DBG_EVENTS * 8) == cudaSuccess) cudaMemset(q, 0, 5 * FF_DBG_FRAMES * FF_DBG_EVENTS * 8);
-      return q;
-    }();
-    static const int exp_flags = [] { const char* e = getenv("SRL_FUSED_EXP"); return e ? atoi(e) : 0; }();
-    EncFusedParams q{obs, p.w1, p.b1, p.w2, p.b2, buf.xs, buf.a1, buf.a2, frames, buf.NF, exp_flags, dbg_buf};
-    g_fused_dbg = dbg_buf;
-    pf.b(PS_ENC_FUSED); SRL_TRY(enc_fused_fwd_launch(q, kPersistentCtas, st)); pf.e(PS_ENC_FUSED);
-    if (wait_before_conv1) SRL_TRY(cudaStreamWaitEvent(st, wait_before_conv1, 0));      // conv3 / fc read the packed weights
-  } else {
   pf.b(PS_S2D); SRL_TRY(launch_s2d(obs, frames, buf.xs, st, p.w1, buf.wpack + WPack::W1K, sp ? buf.wpack_lo + WPack::W1K : nullptr)); pf.e(PS_S2D);
   { RConv1Fwd::Params q{maps.xs_w, maps.w1k, L.w1k, p.b1, buf.a1, buf.a1_lo, frames, buf.NF};
     pf.b(PS_CONV1_FWD); SRL_TRY(res_fwd_launch<RConv1Fwd>(q, cdiv(frames * 441, 128), 2 * kPersistentCtas, st, sp)); pf.e(PS_CONV1_FWD); }
   if (wait_before_conv1) SRL_TRY(cudaStreamWaitEvent(st, wait_before_conv1, 0));      // conv1's weight copy comes from the frame-conversion kernel; conv2 is the first reader of the re-packed copies
   { RConv2Fwd::Params q{maps.a1p0_w, maps.a1p1_w, maps.w2k, L.a1p0_w, L.a1p1_w, L.w2k, p.b2, buf.a2, buf.a2_lo, frames};
     pf.b(PS_CONV2_FWD); SRL_TRY(res_fwd_launch<RConv2Fwd>(q, cdiv(frames * 100, 128), kPersistentCtas, st, sp)); pf.e(PS_CONV2_FWD); }
-  }
   { RConv3Fwd::Params q{maps.a2_w, maps.w3k, L.a2_w, L.w3k, p.b3, buf.a3, buf.a3_lo, frames};
     pf.b(PS_CONV3_FWD); SRL_TRY(res_fwd_launch<RConv3Fwd>(q, cdiv(frames * 81, 128), kPersistentCtas, st, sp)); pf.e(PS_CONV3_FWD); }
   { TFcFwd::Params q{maps.a3m128, maps.wfk, L.a3m128, L.wfk, buf.hpart, frames};
@@ -384,11 +344,6 @@ cudaError_t encoder_forward(const uint8_t* obs, int frames, const ParamPtrs& p, 
     else SRL_TRY((igemm_tma_launch<TFcFwd, 0>(q, dim3(cdiv(frames, 128), 8 * FC_SPLITS), st)));
     pf.e(PS_FC_FWD); }
   return cudaSuccess;
-}
-
-int side_mode() {
-  static const int m = [] { const char* e = getenv("SRL_SIDE_MODE"); return e ? atoi(e) : 0; }();
-  return m;
 }
 
 cudaError_t encoder_backward(const uint8_t* obs, int frames, const EncoderBuffers& buf, const ParamPtrs& g, const TmaMaps& maps, int mode,
@@ -404,8 +359,7 @@ cudaError_t encoder_backward(const uint8_t* obs, int frames, const EncoderBuffer
   // The wgrad GEMMs only feed the optimizer: each runs on its own side stream beside the dgrad chain
   // (dh -> da3 -> da2 -> da1) and beside each other.  With per-kernel profiling on everything stays on `st`.
   const bool fork = ss.side != nullptr && !pf.on;
-  const bool one_side = (side_mode() & 1) != 0;      // diagnostic: all wgrads serial on one side stream
-  cudaStream_t s1 = fork ? ss.side : st, s2 = fork ? (one_side ? ss.side : ss.side2) : st, s3 = fork ? (one_side ? ss.side : ss.side3) : st;
+  cudaStream_t s1 = fork ? ss.side : st, s2 = fork ? ss.side2 : st, s3 = fork ? ss.side3 : st;
   Profiler p1 = pf, p2 = pf, p3 = pf; p1.st = s1; p2.st = s2; p3.st = s3;
   if (do_fc) {
     if (fork) { SRL_TRY(cudaEventRecord(ss.ev[0], st)); SRL_TRY(cudaStreamWaitEvent(s1, ss.ev[0], 0)); }
@@ -431,16 +385,16 @@ cudaError_t encoder_backward(const uint8_t* obs, int frames, const EncoderBuffer
   if (!do_conv) return cudaSuccess;
   if (fork) { SRL_TRY(cudaEventRecord(ss.ev[1], st)); SRL_TRY(cudaStreamWaitEvent(s2, ss.ev[1], 0)); }
   { RConv3Wgrad::Params q{maps.a2_w, maps.da3g_b, L.a2_w, L.da3g_b, buf.wgrad_ws + WS_W3, g.b3, frames * 81, 0};
-    p2.b(PS_CONV3_WGRAD); SRL_TRY(res_wgrad_launch<RConv3Wgrad>(q, side_wgrad_ctas(), s2, sp)); p2.e(PS_CONV3_WGRAD); }
+    p2.b(PS_CONV3_WGRAD); SRL_TRY(res_wgrad_launch<RConv3Wgrad>(q, kSideWgradCtas, s2, sp)); p2.e(PS_CONV3_WGRAD); }
   { RConv3Dgrad::Params q{maps.da3g_w, maps.w3d, L.da3g_w, L.w3d, buf.a2, buf.da2, buf.da2_lo, frames};
-    pf.b(PS_CONV3_DGRAD); SRL_TRY(res_fwd_launch<RConv3Dgrad>(q, cdiv(frames * 81, 128), bwd_ctas(), st, sp)); pf.e(PS_CONV3_DGRAD); }
+    pf.b(PS_CONV3_DGRAD); SRL_TRY(res_fwd_launch<RConv3Dgrad>(q, cdiv(frames * 81, 128), kBwdCtas, st, sp)); pf.e(PS_CONV3_DGRAD); }
   if (fork) { SRL_TRY(cudaEventRecord(ss.ev[2], st)); SRL_TRY(cudaStreamWaitEvent(s3, ss.ev[2], 0)); }
   { RConv2Wgrad::Params q{maps.a1p0_w, maps.a1p1_w, maps.da2g_b, L.a1p0_w, L.a1p1_w, L.da2g_b, buf.wgrad_ws + WS_W2, g.b2, frames * 100, 0};
-    p3.b(PS_CONV2_WGRAD); SRL_TRY(res_wgrad_launch<RConv2Wgrad>(q, side_wgrad_ctas(), s3, sp)); p3.e(PS_CONV2_WGRAD); }
+    p3.b(PS_CONV2_WGRAD); SRL_TRY(res_wgrad_launch<RConv2Wgrad>(q, kSideWgradCtas, s3, sp)); p3.e(PS_CONV2_WGRAD); }
   { RConv2Dgrad::Params q{maps.da2g_w, maps.w2d, L.da2g_w, L.w2d, buf.a1, buf.da1, buf.da1_lo, frames, buf.NF};
-    pf.b(PS_CONV2_DGRAD); SRL_TRY(res_fwd_launch<RConv2Dgrad>(q, cdiv(frames * 100, 128), bwd_ctas(), st, sp)); pf.e(PS_CONV2_DGRAD); }
+    pf.b(PS_CONV2_DGRAD); SRL_TRY(res_fwd_launch<RConv2Dgrad>(q, cdiv(frames * 100, 128), kBwdCtas, st, sp)); pf.e(PS_CONV2_DGRAD); }
   { RConv1Wgrad::Params q{maps.xs_w, maps.da1g_b, L.da1g_b, buf.wgrad_ws + WS_W1, g.b1, frames * 441, 0};
-    pf.b(PS_CONV1_WGRAD); SRL_TRY(res_wgrad_launch<RConv1Wgrad>(q, bwd_ctas(), st, sp)); pf.e(PS_CONV1_WGRAD); }
+    pf.b(PS_CONV1_WGRAD); SRL_TRY(res_wgrad_launch<RConv1Wgrad>(q, kBwdCtas, st, sp)); pf.e(PS_CONV1_WGRAD); }
   if (fork) {      // join: fc wgrad (phase 2 only: phase 1 was joined by the caller of phase 0), conv3 wgrad, conv2 wgrad
     if (do_fc) { SRL_TRY(cudaStreamWaitEvent(st, ss.ev[4], 0)); }
     SRL_TRY(cudaEventRecord(ss.ev[3], s2)); SRL_TRY(cudaStreamWaitEvent(st, ss.ev[3], 0));

@@ -11,20 +11,6 @@ typedef __nv_bfloat16 bf16;
 SRL_DEVINL uint4 ldg16(const void* p) { return __ldg(reinterpret_cast<const uint4*>(p)); }
 SRL_DEVINL uint4 zero16() { return make_uint4(0, 0, 0, 0); }
 
-// 8 consecutive u8 (two aligned u32 words) -> 8 bf16 (exact: 0..255 fit the 8-bit significand)
-SRL_DEVINL uint4 u8x8_to_bf16x8(uint32_t w0, uint32_t w1) {
-  float f[8];
-  f[0] = __uint_as_float(__byte_perm(w0, 0x4B000000u, 0x7540)) - 8388608.f;
-  f[1] = __uint_as_float(__byte_perm(w0, 0x4B000000u, 0x7541)) - 8388608.f;
-  f[2] = __uint_as_float(__byte_perm(w0, 0x4B000000u, 0x7542)) - 8388608.f;
-  f[3] = __uint_as_float(__byte_perm(w0, 0x4B000000u, 0x7543)) - 8388608.f;
-  f[4] = __uint_as_float(__byte_perm(w1, 0x4B000000u, 0x7540)) - 8388608.f;
-  f[5] = __uint_as_float(__byte_perm(w1, 0x4B000000u, 0x7541)) - 8388608.f;
-  f[6] = __uint_as_float(__byte_perm(w1, 0x4B000000u, 0x7542)) - 8388608.f;
-  f[7] = __uint_as_float(__byte_perm(w1, 0x4B000000u, 0x7543)) - 8388608.f;
-  return make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]), pack_bf16x2(f[6], f[7]));
-}
-
 SRL_DEVINL void store_bf16x16(bf16* dst, const float (&v)[16]) {
   uint4 a = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
   uint4 b = make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]), pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));

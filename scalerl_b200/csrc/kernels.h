@@ -10,7 +10,7 @@ namespace srl {
 // per-kernel CUDA-event bracketing (bench.py's roofline numbers): slots of one learner step
 enum ProfSlot { PS_S2D = 0, PS_CONV1_FWD, PS_CONV2_FWD, PS_CONV3_FWD, PS_FC_FWD, PS_HEAD_FWD, PS_TAIL, PS_ZERO_GRADS, PS_HEAD_BWD,
                 PS_FC_WGRAD, PS_FC_DGRAD, PS_CONV3_WGRAD, PS_CONV3_DGRAD, PS_CONV2_WGRAD, PS_CONV2_DGRAD, PS_CONV1_WGRAD,
-                PS_WGRAD_FINALIZE, PS_GRAD_NORM, PS_OPTIMIZER, PS_PACK, PS_ENC_FUSED, PS_COUNT };
+                PS_WGRAD_FINALIZE, PS_GRAD_NORM, PS_OPTIMIZER, PS_PACK, PS_COUNT };
 struct Profiler {
   bool on = false;
   cudaEvent_t* ev = nullptr;   // 2 * PS_COUNT events
@@ -60,7 +60,6 @@ inline cudaError_t ensure_max_dynamic_smem(PerDeviceOnce& once, K kernel, int by
 }
 
 void kstamp_set_encoder(unsigned long long*); void kstamp_set_vtrace(unsigned long long*); void kstamp_set_heads(unsigned long long*);   // diagnostics build (common.cuh)
-int side_mode();   // SRL_SIDE_MODE diagnostic bitmask: 1 = one wgrad side stream, 2 = head wgrad on the main stream, 4 = grad memset on the main stream
 
 struct SideStream {
   cudaStream_t side = nullptr;      // fc wgrad, weight re-pack
@@ -183,14 +182,12 @@ bool make_map(CUtensorMap* m, const void* base, int rank, const uint64_t* dims, 
 cudaError_t build_tma_maps(const EncoderBuffers& buf, int NF, int NB, TmaMaps* maps, const char** why);
 cudaError_t build_tma_maps_lo(const EncoderBuffers& buf, int NF, int NB, TmaMapsLo* maps, const char** why);
 // wpack_lo != nullptr: also the low copies bf16(w - bf16(w)) in the same layouts
-extern unsigned long long* g_fused_dbg;          // SRL_FUSED_DEBUG stamp buffer of the fused encoder front (device memory; 5 x 8 x 8 u64)
 cudaError_t launch_a3_transpose(const __nv_bfloat16* a3, __nv_bfloat16* a3t, int frames, cudaStream_t st);
 cudaError_t launch_pack_weights(const ParamPtrs& p, __nv_bfloat16* wpack, cudaStream_t st, __nv_bfloat16* wpack_lo = nullptr, bool skip_w1k = false);
 // wait_before_conv1: optional event (weight re-pack running on the side stream) that conv1 must wait for
 // mode: 0 = bf16 operands, 1 = fp32-accurate split operands (maps_lo must be valid)
 cudaError_t encoder_forward(const uint8_t* obs, int frames, const ParamPtrs& p, const EncoderBuffers& buf, const TmaMaps& maps, int mode,
-                            cudaStream_t st, const Profiler& pf, cudaEvent_t wait_before_conv1, const TmaMapsLo* maps_lo = nullptr,
-                            bool fused_front = true);      // fused_front: frame conversion + conv1 + conv2 in one kernel (enc_fused.cuh; bf16 mode)
+                            cudaStream_t st, const Profiler& pf, cudaEvent_t wait_before_conv1, const TmaMapsLo* maps_lo = nullptr);
 // backward for the first `frames` frames given buf.dh; accumulates into the (pre-zeroed) gradient tensors in `g`
 // phase: 0 = fc layer only (fc.weight / fc.bias gradients complete and joined to `st` on return: 95 % of the gradient
 //        bytes, ready for an early all-reduce), 1 = conv layers only, 2 = both

@@ -11,7 +11,6 @@
 // H = 513 + A is padded to Hp (multiple of 64); the gate dimension is laid out [4][Hp] so every GEMM has K = Hp or 4Hp.
 // All GEMM operands are bf16 (fp32 accumulate in TMEM); cell state, gate activations and gradients are fp32.
 #include <stdio.h>
-#include <stdlib.h>
 #include <new>
 #include "tma_problems.cuh"
 #include "kernels.h"
@@ -122,369 +121,6 @@ __global__ void lstm_cell_fwd_kernel(const float* __restrict__ gx, const float* 
   if (hm_next) hm_next[i] = __float2bfloat16_rn(done_next[b] ? 0.f : hv);
 }
 
-
-// ------------------------------------------------------------------------------------------------ persistent recurrence (forward)
-// ONE cooperative kernel runs all T1 steps of a layer instead of 2 launches per step (recurrent GEMM + cell kernel):
-//   * CTA c owns hidden units [16c, 16c+16) for all four gates: its 64 gate columns of W_hh (9 K-blocks x [64 rows x 128 B],
-//     73.7 KB bf16) stay in shared memory for the whole scan (one 16-row TMA box per gate and K-block);
-//   * per step: the A operand  m_t . h_{t-1}  (B <= 128 rows x Hp, bf16) streams through a 4-stage TMA ring, 36 tcgen05.mma (N = 64)
-//     accumulate [B x 64] in TMEM, and the epilogue thread of batch row b finishes the LSTM cell for its 16 units -- gx_t + r +
-//     biases, sigma / tanh, done-reset, c_t (kept in REGISTERS across the steps), h_t -- and writes gates / c / h / bf16 h and
-//     next step's operand hm[t+1];
-//   * a grid barrier (atomic counter, 36 co-resident CTAs) separates the steps: hm[t+1] is complete before anybody loads it.
-// Design estimate was ~3 us per step; MEASURED ~15 us (see srl_lstm_create) -- kept opt-in for B <= 128 as the starting point of the
-// next iteration (more epilogue warps, barrier flags instead of an atomic counter).
-constexpr int LREC_THREADS = 192, LREC_STAGES = 4;
-struct LRecFwdParams {
-  SRL_TMAP hm;               // [T1*B][Hp] bf16, box 128 rows x 64
-  SRL_TMAP whh16;            // [4Hp][Hp] bf16, box 16 rows x 64
-  const float* gx;           // [T1*B][4Hp] input projection of every step
-  const float *b_ih, *b_hh;  // [4H]
-  const float* c_init;       // [B][Hp] (padded)
-  const uint8_t* done;       // [T1*B]
-  float *gates, *cseq, *hseq;        // [T1*B][4Hp], [T1*B][Hp], [T1*B][Hp]
-  __nv_bfloat16 *hbf, *hm_out;       // [T1*B][Hp] each (hm_out == the buffer behind the `hm` map)
-  unsigned* counter;         // grid barrier (zeroed before the launch)
-  int T1, B, H, Hp;
-};
-SRL_DEVINL unsigned ld_acquire_gpu(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__global__ void __launch_bounds__(LREC_THREADS, 1) lstm_rec_fwd_kernel(const __grid_constant__ LRecFwdParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int NKB = p.Hp / 64;                                    // 9
-  uint8_t* sW = smem;                                           // NKB x 8192
-  uint8_t* sA = smem + NKB * 8192;                              // LREC_STAGES x 16384
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sA + LREC_STAGES * 16384);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + LREC_STAGES;
-  uint64_t* w_full = bars + 2 * LREC_STAGES;
-  uint64_t* acc_full = w_full + 1;
-  uint64_t* step_go = acc_full + 1;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(step_go + 1);
-  float* s_bias = reinterpret_cast<float*>(tmem_slot + 2);      // [4][16]
-  const int tid = threadIdx.x, warp = tid >> 5, j0 = blockIdx.x * 16;
-  const int G = 4 * p.Hp;
-  if (warp == 4) {
-    if ((tid & 31) == 0) {
-      for (int s = 0; s < LREC_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-      mbar_init(w_full, 1); mbar_init(acc_full, 1); mbar_init(step_go, 1);
-      mbar_fence_init();
-      tma_prefetch_desc(&p.hm); tma_prefetch_desc(&p.whh16);
-    }
-    __syncwarp();
-    tmem_alloc(tmem_slot, 64);
-  }
-  if (tid < 64) {
-    const int q = tid >> 4, j = j0 + (tid & 15);
-    s_bias[tid] = j < p.H ? p.b_ih[q * p.H + j] + p.b_hh[q * p.H + j] : 0.f;
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 4) {
-    if ((tid & 31) == 0) {
-      mbar_arrive_expect_tx(w_full, NKB * 8192);
-      for (int kb = 0; kb < NKB; ++kb)
-        for (int q = 0; q < 4; ++q) tma_load_2d(sW + kb * 8192 + q * 2048, &p.whh16, w_full, kb * 64, q * p.Hp + j0);
-      int n = 0;
-      for (int t = 0; t < p.T1; ++t) {
-        if (t > 0) {
-          mbar_wait(step_go, (t - 1) & 1);                      // every CTA has written its slice of hm[t]
-          asm volatile("fence.proxy.async;" ::: "memory");      // generic-proxy global writes -> visible to the TMA (async proxy) reads
-        }
-        for (int kb = 0; kb < NKB; ++kb, ++n) {
-          const int s = n % LREC_STAGES;
-          mbar_wait(&empty[s], ((n / LREC_STAGES) & 1) ^ 1);
-          mbar_arrive_expect_tx(&full[s], 16384);
-          tma_load_2d(sA + s * 16384, &p.hm, &full[s], kb * 64, t * p.B);
-        }
-      }
-    }
-  } else if (warp == 5) {
-    if ((tid & 31) == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(128, 64, 0, 0);
-      mbar_wait(w_full, 0);
-      int n = 0;
-      for (int t = 0; t < p.T1; ++t) {
-        for (int kb = 0; kb < NKB; ++kb, ++n) {
-          const int s = n % LREC_STAGES;
-          mbar_wait(&full[s], (n / LREC_STAGES) & 1);
-          tc_fence_after();
-          const uint32_t a0 = smem_u32(sA + s * 16384), b0 = smem_u32(sW + kb * 8192);
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_base, make_smem_desc(a0 + k * 32, 16, 1024), make_smem_desc(b0 + k * 32, 16, 1024), idesc, (kb | k) != 0);
-          umma_commit(&empty[s]);
-        }
-        umma_commit(acc_full);
-      }
-    }
-  } else {
-    // ---- epilogue: thread = batch row b; its 16 hidden units' cell state lives in registers for the whole scan
-    const int b = tid;
-    const bool row_ok = b < p.B;
-    const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);
-    float c[16];
-#pragma unroll
-    for (int jj = 0; jj < 16; ++jj) c[jj] = row_ok ? p.c_init[(size_t)b * p.Hp + j0 + jj] : 0.f;
-    for (int t = 0; t < p.T1; ++t) {
-      const size_t row = (size_t)t * p.B + b;
-      // operands of the cell that do not depend on the GEMM: requested before the accumulator is waited for
-      float gxv[4][16];
-      bool dn = false, dn_next = false;
-      if (row_ok) {
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-#pragma unroll
-          for (int v4 = 0; v4 < 4; ++v4) {
-            const float4 x = __ldg(reinterpret_cast<const float4*>(p.gx + row * G + q * p.Hp + j0) + v4);
-            gxv[q][4 * v4] = x.x; gxv[q][4 * v4 + 1] = x.y; gxv[q][4 * v4 + 2] = x.z; gxv[q][4 * v4 + 3] = x.w;
-          }
-        dn = p.done[row] != 0;
-        dn_next = t + 1 < p.T1 ? p.done[row + p.B] != 0 : false;
-      }
-      mbar_wait(acc_full, t & 1);
-      tc_fence_after();
-      uint32_t r[4][16];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) tmem_ld16(lane_base + q * 16, r[q]);
-      tmem_ld_wait();
-      tc_fence_before();
-      if (row_ok) {
-        float hv[16], a[4][16];
-#pragma unroll
-        for (int jj = 0; jj < 16; ++jj) {
-          if (j0 + jj < p.H) {
-            const float pi = __uint_as_float(r[0][jj]) + gxv[0][jj] + s_bias[jj], pf = __uint_as_float(r[1][jj]) + gxv[1][jj] + s_bias[16 + jj];
-            const float pg = __uint_as_float(r[2][jj]) + gxv[2][jj] + s_bias[32 + jj], po = __uint_as_float(r[3][jj]) + gxv[3][jj] + s_bias[48 + jj];
-            a[0][jj] = sigmoidf_(pi); a[1][jj] = sigmoidf_(pf); a[2][jj] = tanhf(pg); a[3][jj] = sigmoidf_(po);
-            const float cp = dn ? 0.f : c[jj];
-            c[jj] = a[1][jj] * cp + a[0][jj] * a[2][jj];
-            hv[jj] = a[3][jj] * tanhf(c[jj]);
-          } else {
-            a[0][jj] = a[1][jj] = a[2][jj] = a[3][jj] = 0.f; c[jj] = 0.f; hv[jj] = 0.f;
-          }
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          float4* o = reinterpret_cast<float4*>(p.gates + row * G + q * p.Hp + j0);
-#pragma unroll
-          for (int v4 = 0; v4 < 4; ++v4) o[v4] = make_float4(a[q][4 * v4], a[q][4 * v4 + 1], a[q][4 * v4 + 2], a[q][4 * v4 + 3]);
-        }
-        float4* oc = reinterpret_cast<float4*>(p.cseq + row * p.Hp + j0);
-        float4* oh = reinterpret_cast<float4*>(p.hseq + row * p.Hp + j0);
-#pragma unroll
-        for (int v4 = 0; v4 < 4; ++v4) {
-          oc[v4] = make_float4(c[4 * v4], c[4 * v4 + 1], c[4 * v4 + 2], c[4 * v4 + 3]);
-          oh[v4] = make_float4(hv[4 * v4], hv[4 * v4 + 1], hv[4 * v4 + 2], hv[4 * v4 + 3]);
-        }
-        store_bf16x16(p.hbf + row * p.Hp + j0, hv);
-        if (t + 1 < p.T1) {
-          float hm[16];
-#pragma unroll
-          for (int jj = 0; jj < 16; ++jj) hm[jj] = dn_next ? 0.f : hv[jj];
-          store_bf16x16(p.hm_out + (row + p.B) * p.Hp + j0, hm);
-        }
-      }
-      if (t + 1 < p.T1) {
-        // grid barrier: all 36 CTAs have written their columns of hm[t+1]
-        __threadfence();
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        if (tid == 0) {
-          atomicAdd(p.counter, 1u);
-          const unsigned target = gridDim.x * (unsigned)(t + 1);
-          unsigned spins = 0;
-          while (ld_acquire_gpu(p.counter) < target) { if (++spins > (1u << 26)) __trap(); }
-          mbar_arrive(step_go);
-        }
-      }
-    }
-  }
-  __syncthreads();
-  if (warp == 4) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 64);
-  }
-}
-
-
-// ------------------------------------------------------------------------------------------------ persistent recurrence (BPTT)
-// One cooperative kernel runs the backward scan t = T-1 .. 0 of a layer.  Per step two phases separated by grid barriers:
-//   A  cell backward for step t: CTA c / thread b own hidden units [16c, 16c+16) of batch row b (as in the forward; the carried
-//      dc stays in registers): dh = dh_out[t] + m_{t+1} . (sum of the 4 K-split partials of dhm_{t+1}) -> dgates_t (bf16);
-//   B  dhm_t = dgates_t . W_hh  ([B x 4Hp] x [4Hp x Hp]) for t > 0: CTA c = (N tile c % 9, K split c / 9) keeps its [64 x 576]
-//      slice of W_hh^T resident in shared memory, streams dgates_t through a TMA ring, 36 tcgen05.mma, and writes its fp32 partial
-//      [B x 64] to dhm_part[split]; the partials are summed (fixed order) by phase A of the next step.
-constexpr int LBWD_SPLITS = 4;
-struct LRecBwdParams {
-  SRL_TMAP dg;               // dgates [T*B][4Hp] bf16, box 128 rows x 64
-  SRL_TMAP whhT;             // W_hh^T [Hp][4Hp] bf16, box 64 rows x 64
-  const float* dh_out;       // [T*B][Hp] gradient w.r.t. the layer's output (fp32, padded)
-  const float *gates, *cseq; // forward activations
-  const float* c_init;       // [B][Hp]
-  const uint8_t* done;       // [T1*B]
-  __nv_bfloat16* dgates;     // [T*B][4Hp] (the buffer behind `dg`)
-  float* dhm_part;           // [LBWD_SPLITS][B][Hp]
-  unsigned* counter;
-  int T, B, H, Hp;
-};
-__global__ void __launch_bounds__(LREC_THREADS, 1) lstm_rec_bwd_kernel(const __grid_constant__ LRecBwdParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int NT = p.Hp / 64, G = 4 * p.Hp, KB = G / 64 / LBWD_SPLITS;       // 9 N tiles, 9 K blocks per split
-  uint8_t* sW = smem;                                           // KB x 8192
-  uint8_t* sA = smem + KB * 8192;                               // LREC_STAGES x 16384
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sA + LREC_STAGES * 16384);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + LREC_STAGES;
-  uint64_t* w_full = bars + 2 * LREC_STAGES;
-  uint64_t* acc_full = w_full + 1;
-  uint64_t* step_go = acc_full + 1;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(step_go + 1);
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const int nt = blockIdx.x % NT, ks = blockIdx.x / NT, j0 = blockIdx.x * 16;
-  if (warp == 4) {
-    if ((tid & 31) == 0) {
-      for (int s = 0; s < LREC_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-      mbar_init(w_full, 1); mbar_init(acc_full, 1); mbar_init(step_go, 1);
-      mbar_fence_init();
-      tma_prefetch_desc(&p.dg); tma_prefetch_desc(&p.whhT);
-    }
-    __syncwarp();
-    tmem_alloc(tmem_slot, 64);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int nsteps = p.T;                 // step index i = 0 .. T-1  <->  t = T-1-i; the GEMM runs for t > 0
-
-  if (warp == 4) {
-    if ((tid & 31) == 0) {
-      mbar_arrive_expect_tx(w_full, KB * 8192);
-      for (int kb = 0; kb < KB; ++kb) tma_load_2d(sW + kb * 8192, &p.whhT, w_full, (ks * KB + kb) * 64, nt * 64);
-      int n = 0;
-      for (int i = 0; i + 1 < nsteps; ++i) {                    // t = T-1-i > 0
-        const int t = p.T - 1 - i;
-        mbar_wait(step_go, i & 1);                              // barrier 1 of this step passed: dgates_t complete
-        asm volatile("fence.proxy.async;" ::: "memory");
-        for (int kb = 0; kb < KB; ++kb, ++n) {
-          const int s = n % LREC_STAGES;
-          mbar_wait(&empty[s], ((n / LREC_STAGES) & 1) ^ 1);
-          mbar_arrive_expect_tx(&full[s], 16384);
-          tma_load_2d(sA + s * 16384, &p.dg, &full[s], (ks * KB + kb) * 64, t * p.B);
-        }
-      }
-    }
-  } else if (warp == 5) {
-    if ((tid & 31) == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(128, 64, 0, 0);
-      mbar_wait(w_full, 0);
-      int n = 0;
-      for (int i = 0; i + 1 < nsteps; ++i) {
-        for (int kb = 0; kb < KB; ++kb, ++n) {
-          const int s = n % LREC_STAGES;
-          mbar_wait(&full[s], (n / LREC_STAGES) & 1);
-          tc_fence_after();
-          const uint32_t a0 = smem_u32(sA + s * 16384), b0 = smem_u32(sW + kb * 8192);
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_base, make_smem_desc(a0 + k * 32, 16, 1024), make_smem_desc(b0 + k * 32, 16, 1024), idesc, (kb | k) != 0);
-          umma_commit(&empty[s]);
-        }
-        umma_commit(acc_full);
-      }
-    }
-  } else {
-    const int b = tid;
-    const bool row_ok = b < p.B;
-    const uint32_t lane_base = tmem_base + ((uint32_t)(warp * 32) << 16);
-    float dc[16];
-#pragma unroll
-    for (int jj = 0; jj < 16; ++jj) dc[jj] = 0.f;
-    auto grid_barrier = [&](unsigned phase) {                   // phase = 1, 2, 3, ...: all CTAs arrived `phase` times
-      __threadfence();
-      asm volatile("bar.sync 1, 128;" ::: "memory");
-      if (tid == 0) {
-        atomicAdd(p.counter, 1u);
-        const unsigned target = gridDim.x * phase;
-        unsigned spins = 0;
-        while (ld_acquire_gpu(p.counter) < target) { if (++spins > (1u << 26)) __trap(); }
-      }
-      asm volatile("bar.sync 1, 128;" ::: "memory");            // everybody sees the other CTAs' writes from here on
-    };
-    unsigned phase = 0;
-    for (int i = 0; i < nsteps; ++i) {
-      const int t = p.T - 1 - i;
-      const size_t row = (size_t)t * p.B + b;
-      // ---- phase A: cell backward of step t for (b, j0 .. j0+15)
-      if (row_ok) {
-        const bool dn = p.done[row] != 0, dn_next = p.done[row + p.B] != 0, have_next = t + 1 < p.T;
-        float d[4][16];
-#pragma unroll
-        for (int jj = 0; jj < 16; ++jj) {
-          const int j = j0 + jj;
-          if (j < p.H) {
-            float dh = p.dh_out[row * p.Hp + j];
-            if (have_next && !dn_next) {
-              float acc = 0.f;
-#pragma unroll
-              for (int sp = 0; sp < LBWD_SPLITS; ++sp) acc += __ldcg(p.dhm_part + ((size_t)sp * p.B + b) * p.Hp + j);
-              dh += acc;
-            }
-            const float* gr = p.gates + row * G + j;
-            const float ig = gr[0], fg = gr[p.Hp], gg = gr[2 * p.Hp], og = gr[3 * p.Hp];
-            const float tc = tanhf(p.cseq[row * p.Hp + j]);
-            const float dct = dh * og * (1.f - tc * tc) + dc[jj];
-            const float cp = dn ? 0.f : (t == 0 ? p.c_init[(size_t)b * p.Hp + j] : p.cseq[(row - p.B) * p.Hp + j]);
-            d[0][jj] = dct * gg * ig * (1.f - ig);
-            d[1][jj] = dct * cp * fg * (1.f - fg);
-            d[2][jj] = dct * ig * (1.f - gg * gg);
-            d[3][jj] = dh * tc * og * (1.f - og);
-            dc[jj] = dn ? 0.f : dct * fg;
-          } else {
-            d[0][jj] = d[1][jj] = d[2][jj] = d[3][jj] = 0.f; dc[jj] = 0.f;
-          }
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) store_bf16x16(p.dgates + row * G + q * p.Hp + j0, d[q]);
-      }
-      if (t == 0) break;                                         // dhm_0 is not needed: no GEMM, no barrier after the last cell
-      grid_barrier(++phase);                                     // barrier 1: dgates_t complete
-      if (tid == 0) mbar_arrive(step_go);
-      // ---- phase B epilogue: this CTA's fp32 partial of dhm_t
-      mbar_wait(acc_full, i & 1);
-      tc_fence_after();
-      uint32_t r[4][16];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) tmem_ld16(lane_base + q * 16, r[q]);
-      tmem_ld_wait();
-      tc_fence_before();
-      if (row_ok) {
-        float4* o = reinterpret_cast<float4*>(p.dhm_part + ((size_t)ks * p.B + b) * p.Hp + nt * 64);
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-#pragma unroll
-          for (int v4 = 0; v4 < 4; ++v4)
-            o[q * 4 + v4] = make_float4(__uint_as_float(r[q][4 * v4]), __uint_as_float(r[q][4 * v4 + 1]), __uint_as_float(r[q][4 * v4 + 2]),
-                                        __uint_as_float(r[q][4 * v4 + 3]));
-      }
-      grid_barrier(++phase);                                     // barrier 2: every partial of dhm_t is written
-    }
-  }
-  __syncthreads();
-  if (warp == 4) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 64);
-  }
-}
-
 // BPTT cell: dh = dh_out[t] + m_{t+1} . dhm_{t+1};  writes dgates (bf16) and the carried dc
 __global__ void lstm_cell_bwd_kernel(const float* __restrict__ dh_out, const float* __restrict__ dhm_next, const uint8_t* __restrict__ done_next,
                                      const float* __restrict__ gates, const float* __restrict__ c_t, const float* __restrict__ c_prev,
@@ -562,10 +198,6 @@ struct srl_lstm {
   float *gx, *r, *gates[2], *cseq[2], *hseq[2], *dc, *dhm, *dx, *dwpad;
   float *h_init, *c_init;    // [2][B][Hp] padded copies
   CUtensorMap m_xin[2], m_hm[2], m_hm64[2], m_xin64[2], m_Wih[2], m_Whh[2], m_WihT[2], m_WhhT[2], m_dg128[2], m_dg64[2];
-  CUtensorMap m_Whh16[2];    // W_hh with 16-row boxes (persistent recurrence: one box per gate and K-block)
-  unsigned* counters;        // grid-barrier counters of the persistent kernels
-  float* dhm_part;           // [LBWD_SPLITS][B][Hp] K-split partials of dhm (persistent BPTT)
-  bool persistent;           // B <= 128 and SRL_LSTM_PERSISTENT != 0
 };
 
 static thread_local char g_lerr[256] = "";
@@ -596,8 +228,7 @@ extern "C" int srl_lstm_create(int T1, int B, int H, const float* const* weights
     o_dg[l] = take(NB * G * 2); o_gates[l] = take(N1 * G * 4); o_c[l] = take(N1 * Hp * 4); o_h[l] = take(N1 * Hp * 4);
   }
   const int64_t o_gx = take(N1 * G * 4), o_r = take((int64_t)B * G * 4), o_dc = take((int64_t)B * Hp * 4), o_dhm = take((int64_t)B * Hp * 4),
-                o_dx = take(NB * Hp * 4), o_dw = take(G * Hp * 4), o_hi = take(2 * (int64_t)B * Hp * 4), o_ci = take(2 * (int64_t)B * Hp * 4),
-                o_cnt = take(256), o_part = take((int64_t)LBWD_SPLITS * B * Hp * 4);
+                o_dx = take(NB * Hp * 4), o_dw = take(G * Hp * 4), o_hi = take(2 * (int64_t)B * Hp * 4), o_ci = take(2 * (int64_t)B * Hp * 4);
   if (cudaMalloc(&L->arena, total) != cudaSuccess || cudaMemset(L->arena, 0, total) != cudaSuccess) { delete L; LREQ(false, "lstm_create: cudaMalloc failed"); }
   char* a = L->arena;
   L->xin[0] = (__nv_bfloat16*)(a + o_xin0);
@@ -610,22 +241,12 @@ extern "C" int srl_lstm_create(int T1, int B, int H, const float* const* weights
   L->xin[1] = L->hbf[0];
   L->gx = (float*)(a + o_gx); L->r = (float*)(a + o_r); L->dc = (float*)(a + o_dc); L->dhm = (float*)(a + o_dhm); L->dx = (float*)(a + o_dx);
   L->dwpad = (float*)(a + o_dw); L->h_init = (float*)(a + o_hi); L->c_init = (float*)(a + o_ci);
-  L->counters = (unsigned*)(a + o_cnt);
-  L->dhm_part = (float*)(a + o_part);
-  // opt-in (SRL_LSTM_PERSISTENT=1): measured SLOWER than the per-step launches on B200 (T1=101, B=128: forward 3.03 vs 2.33 ms, BPTT 6.07
-  // vs 3.88 ms; profiles/r02_lstm_persistent.md) -- ~15 us per step: grid barrier + post-barrier TMA latency + a 16-units-per-thread cell
-  { const char* e = getenv("SRL_LSTM_PERSISTENT"); L->persistent = B <= 128 && e && atoi(e) != 0; }
   bool ok = true;
   for (int l = 0; l < 2 && ok; ++l) {
     ok = ok && map2(&L->m_xin[l], L->xin[l], Hp, N1, 128) && map2(&L->m_xin64[l], L->xin[l], Hp, NB, 64) && map2(&L->m_hm[l], L->hm[l], Hp, N1, 128) &&
          map2(&L->m_hm64[l], L->hm[l], Hp, NB, 64) && map2(&L->m_Wih[l], L->Wih[l], Hp, G, 64) && map2(&L->m_Whh[l], L->Whh[l], Hp, G, 64) &&
          map2(&L->m_WihT[l], L->WihT[l], G, Hp, 64) && map2(&L->m_WhhT[l], L->WhhT[l], G, Hp, 64) && map2(&L->m_dg128[l], L->dgates[l], G, NB, 128) &&
          map2(&L->m_dg64[l], L->dgates[l], G, NB, 64);
-  }
-  for (int l = 0; l < 2 && ok; ++l) {
-    const uint64_t d[2] = {(uint64_t)Hp, (uint64_t)G}, sd[1] = {(uint64_t)Hp};
-    const uint32_t bx[2] = {64, 16};
-    ok = ok && make_map(&L->m_Whh16[l], L->Whh[l], 2, d, sd, bx);
   }
   if (!ok) { cudaFree(L->arena); delete L; LREQ(false, "lstm_create: tensor map creation failed"); }
   *out = L;
@@ -656,16 +277,6 @@ extern "C" int srl_lstm_forward(srl_lstm_t* L, const float* core, const uint8_t*
     lstm_init_hm_kernel<<<cell_blocks, 256, 0, st>>>(h0 + (size_t)l * B * H, done, B, H, Hp, L->hm[l]);
     { LGemmK::Params q{L->m_xin[l], L->m_Wih[l], L->gx, (int)N1, Hp / 64, G, 0, 0};      // input projection of every step
       LCU(igemm_tma_launch<LGemmK>(q, dim3(cdiv_(N1, 128), G / 64), st), "lstm gx gemm"); }
-    if (L->persistent) {
-      LCU(cudaMemsetAsync(L->counters + l, 0, sizeof(unsigned), st), "zero barrier counter");
-      LRecFwdParams q{L->m_hm[l], L->m_Whh16[l], L->gx, L->w[l][2], L->w[l][3], L->c_init + (size_t)l * B * Hp, done, L->gates[l], L->cseq[l],
-                      L->hseq[l], L->hbf[l], L->hm[l], L->counters + l, T1, B, H, Hp};
-      const int smem = (Hp / 64) * 8192 + LREC_STAGES * 16384 + 1024 + 1024;
-      static PerDeviceOnce once;
-      LCU(ensure_max_dynamic_smem(once, lstm_rec_fwd_kernel, smem), "lstm_rec_fwd attr");
-      void* args[] = {&q};
-      LCU(cudaLaunchCooperativeKernel((const void*)lstm_rec_fwd_kernel, dim3(Hp / 16), dim3(LREC_THREADS), args, smem, st), "lstm persistent recurrence");
-    } else
     for (int t = 0; t < T1; ++t) {
       { LGemmK::Params q{L->m_hm[l], L->m_Whh[l], L->r, B, Hp / 64, G, t * B, 0};
         LCU(igemm_tma_launch<LGemmK>(q, dim3(cdiv_(B, 128), G / 64), st), "lstm recurrent gemm"); }
@@ -699,16 +310,6 @@ extern "C" int srl_lstm_backward(srl_lstm_t* L, const float* dout, const uint8_t
   LCU(cudaMemcpy2DAsync(L->dx, Hp * 4, dout, H * 4, H * 4, NB, cudaMemcpyDeviceToDevice, st), "pad dout");
   for (int l = 1; l >= 0; --l) {
     LCU(cudaMemsetAsync(L->dc, 0, (size_t)B * Hp * 4, st), "zero dc");
-    if (L->persistent && G / 64 % LBWD_SPLITS == 0 && (Hp / 64) * LBWD_SPLITS == Hp / 16) {
-      LCU(cudaMemsetAsync(L->counters + 2 + l, 0, sizeof(unsigned), st), "zero barrier counter");
-      LRecBwdParams q{L->m_dg128[l], L->m_WhhT[l], L->dx, L->gates[l], L->cseq[l], L->c_init + (size_t)l * B * Hp, done, L->dgates[l], L->dhm_part,
-                      L->counters + 2 + l, T, B, H, Hp};
-      const int smem = (G / 64 / LBWD_SPLITS) * 8192 + LREC_STAGES * 16384 + 1024 + 1024;
-      static PerDeviceOnce once;
-      LCU(ensure_max_dynamic_smem(once, lstm_rec_bwd_kernel, smem), "lstm_rec_bwd attr");
-      void* args[] = {&q};
-      LCU(cudaLaunchCooperativeKernel((const void*)lstm_rec_bwd_kernel, dim3(Hp / 16), dim3(LREC_THREADS), args, smem, st), "lstm persistent BPTT");
-    } else
     for (int t = T - 1; t >= 0; --t) {
       const float* cprev = t == 0 ? L->c_init + (size_t)l * B * Hp : L->cseq[l] + (size_t)(t - 1) * B * Hp;
       lstm_cell_bwd_kernel<<<cell_blocks, 256, 0, st>>>(

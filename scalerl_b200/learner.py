@@ -554,13 +554,11 @@ class B200ImpalaLearner(BaseAgent):
         dist = torch.distributed
         fcw = self.flat_grads[self._off[6]:]
         small = self.flat_grads[:self._off[6]]
-        skip = bool(os.environ.get('SRL_DP_SKIP_ALLREDUCE'))      # diagnostics only: measures the cost of the split itself
         begin()
-        work = None if skip else dist.all_reduce(fcw, op=dist.ReduceOp.SUM, group=self.pg or None, async_op=True)
+        work = dist.all_reduce(fcw, op=dist.ReduceOp.SUM, group=self.pg or None, async_op=True)
         finish()
-        if not skip:
-            dist.all_reduce(small, op=dist.ReduceOp.SUM, group=self.pg or None)
-            work.wait()
+        dist.all_reduce(small, op=dist.ReduceOp.SUM, group=self.pg or None)
+        work.wait()
         apply()
 
     def release_graphs(self):
@@ -605,28 +603,13 @@ class B200ImpalaLearner(BaseAgent):
                 with torch.cuda.graph(g[1], stream=self._capture_stream()):
                     self.apply_gradients()
             elif self._dist:
-                g = None
-                if os.environ.get('SRL_DP_SINGLE_GRAPH'):
-                    try:        # opt-in: ONE graph with the two NCCL all-reduces captured inside it (measured: no faster than split
-                                # graphs, and process-group teardown can hang while such graphs are alive -- call release_graphs() first)
-                        g1 = torch.cuda.CUDAGraph()
-                        with torch.cuda.graph(g1, stream=self._capture_stream()):
-                            self._dp_step(batch, lambda: self.forward_backward_begin(batch), lambda: self.backward_finish(batch),
-                                          self.apply_gradients)
-                        g = (g1,)
-                    except Exception as e:     # e.g. an NCCL build that cannot be stream-captured
-                        import warnings
-                        warnings.warn(f'capturing NCCL inside the step graph failed ({e!r}); falling back to split graphs')
-                        torch.cuda.synchronize()
-                        g = None
-                if g is None:
-                    g = tuple(torch.cuda.CUDAGraph() for _ in range(3))
-                    with torch.cuda.graph(g[0], stream=self._capture_stream()):
-                        self.forward_backward_begin(batch)
-                    with torch.cuda.graph(g[1], stream=self._capture_stream()):
-                        self.backward_finish(batch)
-                    with torch.cuda.graph(g[2], stream=self._capture_stream()):
-                        self.apply_gradients()
+                g = tuple(torch.cuda.CUDAGraph() for _ in range(3))
+                with torch.cuda.graph(g[0], stream=self._capture_stream()):
+                    self.forward_backward_begin(batch)
+                with torch.cuda.graph(g[1], stream=self._capture_stream()):
+                    self.backward_finish(batch)
+                with torch.cuda.graph(g[2], stream=self._capture_stream()):
+                    self.apply_gradients()
             else:
                 g = (torch.cuda.CUDAGraph(),)
                 with torch.cuda.graph(g[0], stream=self._capture_stream()):

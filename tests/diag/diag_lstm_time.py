@@ -1,5 +1,5 @@
-"""LSTM core alone (srl_lstm_forward / srl_lstm_backward), persistent recurrence kernels vs one launch pair per step.
-    python tests/diag/diag_lstm_time.py [T1 B A]        (run once per SRL_LSTM_PERSISTENT = 1 / 0)"""
+"""LSTM core alone (srl_lstm_forward / srl_lstm_backward, one launch pair per step), each replayed as a CUDA graph.
+    python tests/diag/diag_lstm_time.py [T1 B A]"""
 import os
 import sys
 
@@ -35,7 +35,7 @@ def main():
             g1.replay()
         b.record(); torch.cuda.synchronize()
         res[name] = a.elapsed_time(b) / 5
-    print(f'SRL_LSTM_PERSISTENT={os.environ.get("SRL_LSTM_PERSISTENT", "1")} T1={T1} B={B} H={H}: forward {res["forward"]:.3f} ms  backward {res["backward"]:.3f} ms'
+    print(f'T1={T1} B={B} H={H}: forward {res["forward"]:.3f} ms  backward {res["backward"]:.3f} ms'
           f'  checksum {float(out.double().sum()):.6f} {float(core.grads["rnn_layer.weight_hh_l0"].double().sum()):.6f}')
 
 

@@ -22,7 +22,7 @@ with ctx:
         da1 = L.debug_buffer('da1').float().view(-1, 32)
         d1.append(da1.sum(0).clone())
         torch.cuda.synchronize()
-tag = 'PDL=%s MASK=%s SIDE=%s STREAM=%s' % tuple(os.environ.get(k, '-') for k in ('SRL_PDL', 'SRL_PDL_MASK', 'SRL_SIDE_MODE', 'DIAG_STREAM'))
+tag = 'PDL=%s MASK=%s STREAM=%s' % tuple(os.environ.get(k, '-') for k in ('SRL_PDL', 'SRL_PDL_MASK', 'DIAG_STREAM'))
 nbad = 0
 for it in range(N):
     bad = {k: float((gs[it][k] - gs[0][k]).norm() / gs[0][k].norm()) for k in gs[0]}

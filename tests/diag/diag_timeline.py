@@ -15,7 +15,7 @@ from scalerl_b200.learner import B200ImpalaLearner, ImpalaHParams   # noqa: E402
 NAMES = {1: 'obs_s2d', 2: 'pack_weights', 11: 'conv1_fwd', 12: 'conv2_fwd', 13: 'conv3_fwd', 14: 'conv3_dgrad', 15: 'conv2_dgrad',
          21: 'conv3_wgrad', 22: 'conv2_wgrad', 23: 'conv1_wgrad', 31: 'fc_fwd', 32: 'fc_dgrad', 33: 'fc_wgrad', 34: 'lstm_gemm_k', 35: 'lstm_gemm_mn', 36: 'fc_wgrad',
          41: 'column_step', 44: 'impala_tail', 45: 'impala_tail_warp', 46: 'head_fwd', 47: 'head_bwd_dh', 48: 'head_wgrad', 51: 'conv_wgrad_finalize',
-         52: 'clip_optim', 53: 'a3_transpose', 54: 'enc_fused_fwd'}
+         52: 'clip_optim', 53: 'a3_transpose'}
 T, B = (int(sys.argv[1]), int(sys.argv[2])) if len(sys.argv) > 2 else (20, 32)
 A = 6
 L = B200ImpalaLearner(ImpalaHParams(rollout_length=T, batch_size=B, num_actions=A), init_state_dict=O.init_params(A, seed=1), process_group=False)

@@ -1,6 +1,6 @@
 """One small learner step of every kernel family, eager launches -- the workload for compute-sanitizer (tools/sanitize.sh):
     compute-sanitizer --tool memcheck|racecheck|synccheck|initcheck python tests/diag/sanitize_step.py [mode ...]
-modes: bf16 (default step), fused (SRL_FUSED_FWD=1 front kernel), split (fp32-accurate operands), three (no column fusion), lstm, ops"""
+modes: bf16 (default step), split (fp32-accurate operands), three (no column fusion), lstm, ops"""
 import os
 import sys
 
@@ -27,12 +27,10 @@ def step(tag, T=3, B=5, A=6, state=False, **kw):
 
 
 def main():
-    modes = sys.argv[1:] or ['bf16', 'fused', 'split', 'three', 'lstm', 'ops']
+    modes = sys.argv[1:] or ['bf16', 'split', 'three', 'lstm', 'ops']
     if 'bf16' in modes:
         step('bf16')
         step('bf16 adam', optimizer='adam')
-    if 'fused' in modes:
-        step('fused front', opts={'fused_fwd': 1})
     if 'split' in modes:
         step('fp32_split', precision='fp32_split')
     if 'three' in modes:
